@@ -13,8 +13,8 @@ With N > 1 the per-GPU batch is BASELINE configs[2]'s shard (65 536 rays / 8 = 8
 
 Prints ONE JSON line on rank 0 (see the task contract): value = ray-samples/s with inputs resident in HBM
 (device-timed with CUDA events), e2e = the same through the public API from pinned host buffers including
-H2D/D2H, roofline for the dominant (MLP) kernel, cpu_baseline = the UNMODIFIED reference (baseline/_ref, see
-baseline/README.md; `kind: "reference"`) timed on the host cores - the oracle port (`kind: "port"`) when _ref is absent.
+H2D/D2H, roofline for the dominant (MLP) kernel, cpu_baseline = the oracle port of the reference (`kind: "port"`) timed on
+the host cores.
 """
 from __future__ import annotations
 
@@ -67,64 +67,8 @@ def peaks():
     return dict(tflops=1590.0, tflops_sustained=1400.0, hbm=6650.0, src='fallback')
 
 
-# ------------------------------------------------------------------------------------------------
-# The unmodified reference (baseline/_ref/mega_nerf, a copy of /root/reference/mega_nerf made by baseline/make_ref.py)
-# ------------------------------------------------------------------------------------------------
-_REF = None
-
-
-def load_reference():
-    """-> namespace with the reference's own render_rays / NeRF / MegaNeRF / Cascade / ShiftedSoftplus, or None."""
-    global _REF
-    if _REF is not None:
-        return _REF or None
-    ref_root = os.path.join(ROOT, 'baseline', '_ref')
-    if os.environ.get('MN_BENCH_NO_REF') == '1' or not os.path.isdir(os.path.join(ref_root, 'mega_nerf')):
-        _REF = False
-        return None
-    try:
-        sys.path.insert(0, ref_root)
-        from mega_nerf.rendering import render_rays
-        from mega_nerf.models.nerf import NeRF, ShiftedSoftplus
-        from mega_nerf.models.mega_nerf import MegaNeRF
-        from mega_nerf.models.cascade import Cascade
-        import mega_nerf
-        _REF = Namespace(render_rays=render_rays, NeRF=NeRF, ShiftedSoftplus=ShiftedSoftplus, MegaNeRF=MegaNeRF,
-                         Cascade=Cascade, path=os.path.dirname(mega_nerf.__file__))
-    except Exception as e:  # noqa: BLE001
-        log(f'baseline/_ref present but not importable ({e!r}); falling back to the oracle port')
-        _REF = False
-    finally:
-        if ref_root in sys.path:
-            sys.path.remove(ref_root)
-    return _REF or None
-
-
-def reference_net(R, net, device='cpu'):
-    """The reference's own modules (models/nerf.py:45, mega_nerf.py:7, cascade.py:7) holding the workload's weights."""
-    spec = net.spec
-    subs = []
-    for w in net.weights:
-        m = R.NeRF(spec.pos_xyz_dim, spec.pos_dir_dim, spec.layers, list(spec.skip_layers), spec.layer_dim, spec.appearance_dim,
-                   spec.affine_appearance, spec.appearance_count, spec.rgb_dim, spec.xyz_dim,
-                   R.ShiftedSoftplus() if spec.shifted_softplus else torch.nn.ReLU())
-        m.load_state_dict(w)
-        subs.append(m)
-    if net.kind == 'nerf':
-        out = subs[0]
-    elif net.kind == 'cascade':
-        out = R.Cascade(subs[0], subs[1])
-    else:
-        out = R.MegaNeRF(subs, net.centroids.clone(), net.boundary_margin, net.xyz_real, net.cluster_2d)
-    return out.to(device).eval()
-
-
 def cpu_renderer(O, net, opts):
-    """-> (fn(rays, idx) -> results, kind): the reference itself when baseline/_ref is there, else the oracle port."""
-    R = load_reference()
-    if R is not None:
-        rnet, hp = reference_net(R, net), Namespace(**vars(opts))
-        return (lambda r, i: R.render_rays(rnet, None, r, i, hp, None, None, True, False, False)[0]), 'reference'
+    """-> (fn(rays, idx) -> results, kind): the oracle port of the reference's render_rays."""
     return (lambda r, i: O.render_rays(net, None, r, i, opts, None, None, True, False, False)[0]), 'port'
 
 
@@ -239,9 +183,8 @@ def cpu_rays_per_sec(render, rays, idx, n_probe: int = 64) -> float:
 
 
 def run_reference(args, rank: int):
-    """The reference's own CPU implementation of the path on the host cores: the unmodified mega_nerf.rendering.render_rays
-    + mega_nerf.models from baseline/_ref (kind "reference"); the oracle port of it (oracle/mn_oracle.py, kind "port") only
-    when _ref is absent."""
+    """The reference algorithm on the host cores: the oracle port of mega_nerf.rendering.render_rays + mega_nerf.models
+    (oracle/mn_oracle.py, kind "port")."""
     if rank != 0:
         return
     from oracle import mn_oracle as O
@@ -268,8 +211,7 @@ def run_reference(args, rank: int):
         'config': {'workload': workload_string(), 'cpu_sample': f'each CPU step renders a {sample}-ray sample of it'},
         'cpu_baseline': {'value': value, 'unit': 'samples/s', 'cores': torch.get_num_threads(), 'kind': kind,
                          'sample': f'{sample} of {N_RAYS} rays per step, {args.steps} steps',
-                         'what': ('unmodified mega_nerf.rendering.render_rays + mega_nerf.models (baseline/_ref), torch CPU fp32, '
-                                  'inference_mode' if kind == 'reference' else 'oracle port (baseline/_ref absent)')},
+                         'what': 'oracle port of mega_nerf.rendering.render_rays + mega_nerf.models, torch CPU fp32, inference_mode'},
         'e2e': {'value': value, 'unit': 'samples/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }
@@ -277,23 +219,16 @@ def run_reference(args, rank: int):
 
 
 def gpu_incumbent(O, net, rays_d, idx_d, opts, dev, steps: int = 5):
-    """SURVEY.md §8d "GPU incumbent": the UNMODIFIED reference (baseline/_ref: mega_nerf.rendering.render_rays over
-    mega_nerf.models, i.e. cuBLAS GEMMs + ~10^3 ATen elementwise launches per step) through torch-CUDA on the SAME B200
-    in the three precisions it can run in - fp32, TF32, and autocast fp16 (its default, runner.py:243); the oracle
-    restatement moved to CUDA when _ref is absent.  A baseline leg like cpu_baseline: reported next to the product's
-    number, never on the product path.  Any failure is reported, not raised."""
-    R = load_reference()
-    out = {'kind': 'reference (baseline/_ref under torch-CUDA eager, same GPU)' if R is not None else
-                   'port (oracle restatement under torch-CUDA eager, same GPU)', 'unit': 'samples/s', 'steps': steps}
+    """SURVEY.md §8d "GPU incumbent": the oracle restatement of the reference's render_rays over mega_nerf.models (cuBLAS
+    GEMMs + ~10^3 ATen elementwise launches per step) through torch-CUDA on the SAME B200 in the three precisions the
+    reference can run in - fp32, TF32, and autocast fp16 (its default, runner.py:243).  A baseline leg like cpu_baseline:
+    reported next to the product's number, never on the product path.  Any failure is reported, not raised."""
+    out = {'kind': 'port (oracle restatement under torch-CUDA eager, same GPU)', 'unit': 'samples/s', 'steps': steps}
     try:
         n = rays_d.shape[0]
         samples = n * (opts.coarse_samples + opts.fine_samples)
-        if R is not None:
-            rnet, hp = reference_net(R, net, dev), Namespace(**vars(opts))
-            render = lambda: R.render_rays(rnet, None, rays_d, idx_d, hp, None, None, True, False, False)   # noqa: E731
-        else:
-            netd = O.net_to(net, dev)
-            render = lambda: O.render_rays(netd, None, rays_d, idx_d, opts, None, None, True, False, False)  # noqa: E731
+        netd = O.net_to(net, dev)
+        render = lambda: O.render_rays(netd, None, rays_d, idx_d, opts, None, None, True, False, False)  # noqa: E731
         saved = (torch.backends.cuda.matmul.allow_tf32, torch.backends.cudnn.allow_tf32)
         for name, tf32, amp in (('fp32', False, False), ('tf32', True, False), ('amp_fp16', True, True)):
             torch.backends.cuda.matmul.allow_tf32 = tf32
@@ -317,6 +252,19 @@ def gpu_incumbent(O, net, rays_d, idx_d, opts, dev, steps: int = 5):
     except Exception as e:  # noqa: BLE001
         out['error'] = repr(e)[:300]
     return out
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: every array as out_dir/<name>.npy in float32, so that two builds can be compared output for output."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items() if torch.is_tensor(v)}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit(f'--dump-outputs: {total} bytes of outputs exceed 64 MiB')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), a)
+    log(f'outputs of the last timed step: {sorted(arrays)} -> {out_dir}')
 
 
 def log(msg):
@@ -532,7 +480,12 @@ def main():
                     help="'render' = the graded line; 'train' = one optimisation step (forward + backward + Adam) of the same "
                          "workload through the recording path (SURVEY.md §8f-1); 'cluster' = the cluster-mask kernel on one "
                          "48k-ray chunk x 1000 samples (SURVEY.md §8f-3); both diagnostics only")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='render mode: write the results of the last timed step (and, when N > 1, the all-gathered '
+                         '[rays, 4] buffer) as DIR/<name>.npy in float32; the inputs are seeded, identical from run to run')
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != 'b200' or args.mode != 'render'):
+        ap.error('--dump-outputs applies to the render mode of --impl b200')
     rank = int(os.environ.get('RANK', '0'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -623,6 +576,8 @@ def main():
                 dist.all_gather_into_tensor(gather_buf, packed)
         out_pin.copy_(packed, non_blocking=True)
 
+    last = {}                                   # what the most recent timed step returned
+
     def timed(fn, steps):
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         if world > 1:
@@ -631,7 +586,7 @@ def main():
         for a, b in evs:
             flush.fill_(1)                      # L2 flush between timed iterations (not timed)
             a.record()
-            fn()
+            last['out'] = fn()
             b.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -670,6 +625,12 @@ def main():
     if rank == 0:
         sampler.start()
     ms_total = timed(step_resident, args.steps)
+    if args.dump_outputs and rank == 0:
+        # copied now: the next graph replay overwrites the static result buffers
+        outs = dict(last['out'])
+        if world > 1:
+            outs['gathered'] = pg.buf if pg is not None else gather_buf
+        dump_outputs(args.dump_outputs, outs)
     launches = launches_per_step * args.steps
     samples_per_step = N_RAYS * (COARSE + FINE) * world
     value = samples_per_step * args.steps / (ms_total * 1e-3)
@@ -750,20 +711,17 @@ def main():
         log(f'parity: rgb {par_rgb:.2e} depth {par_depth:.2e}' + (f' gathered rgb {par_g_rgb:.2e} depth {par_g_depth:.2e}' if world > 1 else ''))
         cpu = None
         if world == 1 and not args.no_cpu_baseline:
-            # the reference's own CPU path (baseline/_ref; oracle port when absent) on a bounded sample of the same batch
+            # the reference algorithm's CPU path (oracle port) on a bounded sample of the same batch
             torch.set_num_threads(usable_cpus())
             render_cpu, cpu_kind = cpu_renderer(O, net, opts)
             rate = cpu_rays_per_sec(render_cpu, rays_h, idx_h)
             n_cpu = int(min(N_RAYS, max(64, rate * 15.0))) // 64 * 64         # ~15 s of CPU work
             with torch.inference_mode():
                 t0 = time.perf_counter()
-                ref_out = render_cpu(rays_h[:n_cpu], idx_h[:n_cpu])
+                render_cpu(rays_h[:n_cpu], idx_h[:n_cpu])
                 dt = time.perf_counter() - t0
             cpu = {'value': n_cpu * (COARSE + FINE) / dt, 'unit': 'samples/s', 'cores': torch.get_num_threads(),
                    'kind': cpu_kind, 'sample': f'first {n_cpu} of the {N_RAYS} rays of the same batch ({dt:.1f} s), after a 64-ray probe'}
-            if cpu_kind == 'reference':
-                # the checker itself against the unmodified reference on this box (bit-exact in the build container)
-                cpu['oracle_vs_reference_max_abs_rgb'] = float((ref_out['rgb_fine'][:N_PAR] - ref_rgb).abs().max())
             log(f'cpu baseline ({cpu_kind}): {cpu["value"]:.3e} samples/s on {cpu["cores"]} threads')
 
         line = {

@@ -1,4 +1,5 @@
-"""GPU: the reference's OWN Runner (baseline/_ref/mega_nerf/runner.py, unmodified) on top of mega_nerf_b200.install():
+"""GPU: the reference's OWN Runner (mega_nerf/runner.py of the reference checkout that MEGA_NERF_REFERENCE names, unmodified;
+skipped without one) on top of mega_nerf_b200.install():
 `Runner.render_image` (runner.py:540-578, the eval path: get_ray_directions -> get_rays -> chunked render_rays with
 get_depth / get_bg_fg_rgb) and one `Runner._training_step` (runner.py:347-378) + backward, compared with the same Runner
 on the reference's unmodified hot path (torch-CUDA fp32, TF32 off) on the same synthetic dataset directory, same seed.
@@ -14,7 +15,7 @@ import torch
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref')
+REF = os.environ.get('MEGA_NERF_REFERENCE', '')
 
 CHILD = r'''
 import os, sys, math
@@ -104,7 +105,7 @@ def run_side(mode, variant, ds, out):
     return torch.load(os.path.join(out, mode + '.pt'), map_location='cpu', weights_only=False)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'mega_nerf')), reason='baseline/_ref (copy of the reference package, baseline/make_ref.py) not present')
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'mega_nerf')), reason='needs a reference checkout named by MEGA_NERF_REFERENCE')
 @pytest.mark.parametrize('variant', ['bg', 'nobg'])
 def test_reference_runner_on_top_of_install(tmp_path, variant):
     ds, out = str(tmp_path / 'dataset'), str(tmp_path / 'out')

@@ -1,9 +1,10 @@
 """GPU: loader-side ray generation (SURVEY.md §8f-6).  `get_rays_pairs` against the oracle's get_rays_batch product gathered at
-the same (image, pixel) pairs, and `mega_nerf_b200.loader._load_chunk_inner` against the reference's own
-`FilesystemDataset._load_chunk_inner` (baseline/_ref, unbound method on the same stand-in dataset object and the same parquet
-chunk written with pyarrow in the reference's column layout, filesystem_dataset.py:95-131,222-260)."""
+the same (image, pixel) pairs, and `mega_nerf_b200.loader._load_chunk_inner` against what the reference's own
+`FilesystemDataset._load_chunk_inner` returned for the same stand-in dataset object and the same parquet chunk in the
+reference's column layout (filesystem_dataset.py:95-131,222-260), stored in tests/golden/loader_chunk_v1.pt by
+tests/golden/make_loader_chunk.py."""
+import hashlib
 import os
-import sys
 import types
 from itertools import cycle
 from pathlib import Path
@@ -17,7 +18,9 @@ from test_gpu_parity import DEV, M
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'baseline', '_ref')
+CHUNK_GOLDEN_PATH = os.path.join(ROOT, 'tests', 'golden', 'loader_chunk_v1.pt')
+RAY_CHUNK_SIZE = 64 * 1024                                               # the reference loader's rays per get_rays_batch call
+NEAR, FAR, ALT = 0.1, 3.0, [-0.35, 0.05]
 
 
 def scene(n_img=7, W=13, H=9):
@@ -55,37 +58,46 @@ def test_rays_pairs_bad_index_raises():
         K.check(K.lib().mn_check_status(K.ctx(DEV), K.stream_of(DEV)), K.ctx(DEV))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'mega_nerf')), reason='baseline/_ref not present')
-def test_chunk_loader_matches_reference_method(tmp_path):
-    import numpy as np
-    import pyarrow as pa
-    import pyarrow.parquet as pq
-    from ref_shims import install_shims
-    install_shims()
-    sys.path.insert(0, REF)
-    try:
-        from mega_nerf.datasets.filesystem_dataset import FilesystemDataset     # unmodified reference class
-    finally:
-        sys.path.remove(REF)
-    assert FilesystemDataset._load_chunk_inner.__module__ == 'mega_nerf.datasets.filesystem_dataset'
+def chunk_case():
+    """-> (directions, c2ws, img_indices, pixel_indices, rgbs as uint8) of one seeded parquet chunk"""
     dirs, c2w, g = scene(n_img=5, W=16, H=10)
     rows = 70000                                                          # > RAY_CHUNK_SIZE: the reference loops twice
     img = torch.randint(0, c2w.shape[0], (rows,), generator=g, dtype=torch.int32)
     pix = torch.randint(0, dirs.shape[0], (rows,), generator=g, dtype=torch.int32)
     rgb = torch.randint(0, 256, (rows, 3), generator=g, dtype=torch.uint8)
-    path = tmp_path / 'chunk0.parquet'
+    return dirs, c2w, img, pix, rgb
+
+
+def write_chunk(path, img, pix, rgb):
+    import pyarrow as pa
+    import pyarrow.parquet as pq
     cols = {'img_indices': pa.array(img.numpy()), 'pixel_indices': pa.array(pix.numpy())}
     for c in range(3):
         cols[f'rgbs_{c}'] = pa.array(rgb[:, c].numpy())
     pq.write_table(pa.table(cols), path)
 
-    def dataset():
-        return types.SimpleNamespace(_chunk_index=cycle(range(1)), _parquet_paths=[Path(path)], _directions=dirs.to(DEV), _c2ws=c2w,
-                                     _device=DEV, _near=0.1, _far=3.0, _ray_altitude_range=[-0.35, 0.05])
-    want = FilesystemDataset._load_chunk_inner(dataset())                    # reference: get_rays_batch product + .cpu() + gather
+
+def chunk_dataset(path, dirs, c2w, device):
+    """the attributes of a FilesystemDataset that _load_chunk_inner reads"""
+    return types.SimpleNamespace(_chunk_index=cycle(range(1)), _parquet_paths=[Path(path)], _directions=dirs.to(device), _c2ws=c2w,
+                                 _device=device, _near=NEAR, _far=FAR, _ray_altitude_range=ALT)
+
+
+def digest(t: torch.Tensor) -> str:
+    return hashlib.sha256(t.contiguous().numpy().tobytes()).hexdigest()
+
+
+def test_chunk_loader_matches_reference_method(tmp_path):
+    dirs, c2w, img, pix, rgb = chunk_case()
+    path = tmp_path / 'chunk0.parquet'
+    write_chunk(path, img, pix, rgb)
+    want = torch.load(CHUNK_GOLDEN_PATH, map_location='cpu', weights_only=False)
     from mega_nerf_b200 import loader
-    got = loader._load_chunk_inner(dataset())
-    assert got[0] == want[0]
-    assert torch.equal(got[1], want[1]) and torch.equal(got[3], want[3])
-    assert got[2].shape == want[2].shape and got[2].device.type == 'cpu'
-    assert float((got[2] - want[2]).abs().max()) <= 2e-6                  # torch-CUDA matmul vs the FMA chain of mn_rays
+    got = loader._load_chunk_inner(chunk_dataset(path, dirs, c2w, DEV))
+    assert got[0] == str(path)
+    assert digest(got[1]) == want['rgbs_sha256'] and digest(got[3]) == want['img_indices_sha256']
+    assert got[2].shape == (img.shape[0], 8) and got[2].device.type == 'cpu'
+    # the reference's ray of every row: its (get_rays_batch call, image, pixel) entry of the stored table
+    rows = torch.arange(img.shape[0])
+    ref_rays = want['rays_by_pair'][rows // RAY_CHUNK_SIZE, img.long(), pix.long()]
+    assert float((got[2] - ref_rays).abs().max()) <= 2e-6                 # torch matmul vs the FMA chain of mn_rays

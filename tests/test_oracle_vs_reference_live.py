@@ -1,12 +1,13 @@
-"""CPU-only, build container only (skipped where /root/reference is absent, e.g. on the GPU box): randomised
-configurations - widths, depths, skip layers, SH degree, appearance / affine, cascade, background, routing margin,
-2-D / 3-D clustering, train / eval mode - rendered by the UNMODIFIED reference (imported read-only) and by the oracle
-with the same seeds.  Results and parameter gradients must agree bit for bit.  This is the live form of the pinning that
-the committed fixtures freeze (tests/golden/*.pt)."""
+"""CPU-only: randomised configurations - widths, depths, skip layers, SH degree, appearance / affine, cascade, background,
+routing margin, 2-D / 3-D clustering, train / eval mode - rendered by the oracle with the same seeds as the UNMODIFIED
+reference was, whose results and parameter gradients (tests/golden/reference_live_v1.pt, written by
+tests/golden/make_reference_live.py) they must match bit for bit; and the reference's call surface (signatures, state-dict
+layouts) that the product's drop-in symbols must reproduce."""
 import dataclasses
+import hashlib
+import inspect
 import os
 import random
-import sys
 
 import pytest
 import torch
@@ -14,15 +15,42 @@ import torch
 import cases as C
 from oracle import mn_oracle as O
 
-REF = os.environ.get('MEGA_NERF_REFERENCE', '/root/reference')
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'mega_nerf')), reason='reference checkout not present')
+GOLDEN_PATH = os.path.join(C.ROOT, 'tests', 'golden', 'reference_live_v1.pt')
+SEEDS = list(range(16))
+# (symbol of mega_nerf_b200, the reference symbol it replaces as 'module:qualname')
+SURFACE = [('render_rays', 'mega_nerf.rendering:render_rays'), ('get_rays', 'mega_nerf.ray_utils:get_rays'),
+           ('get_rays_batch', 'mega_nerf.ray_utils:get_rays_batch'),
+           ('get_ray_directions', 'mega_nerf.ray_utils:get_ray_directions'),
+           ('eval_sh', 'mega_nerf.spherical_harmonics:eval_sh'),
+           ('NeRF.__init__', 'mega_nerf.models.nerf:NeRF.__init__'), ('NeRF.forward', 'mega_nerf.models.nerf:NeRF.forward'),
+           ('MegaNeRF.__init__', 'mega_nerf.models.mega_nerf:MegaNeRF.__init__'),
+           ('MegaNeRF.forward', 'mega_nerf.models.mega_nerf:MegaNeRF.forward'),
+           ('Cascade.__init__', 'mega_nerf.models.cascade:Cascade.__init__'),
+           ('Cascade.forward', 'mega_nerf.models.cascade:Cascade.forward'),
+           ('Embedding.__init__', 'mega_nerf.models.nerf:Embedding.__init__'),
+           ('ShiftedSoftplus.__init__', 'mega_nerf.models.nerf:ShiftedSoftplus.__init__')]
+STATE_DICT_KINDS = ('nerf', 'cascade', 'mega')
+STATE_DICT_SPEC = O.NerfSpec(layer_dim=32, appearance_count=5)
 
 
 @pytest.fixture(scope='module')
-def MG():
-    sys.path.insert(0, os.path.join(C.ROOT, 'tests', 'golden'))
-    import make_golden
-    return make_golden
+def live():
+    return torch.load(GOLDEN_PATH, map_location='cpu', weights_only=False)
+
+
+def signature_of(fn):
+    """[(name, repr(default), kind)] of every parameter."""
+    return [(p.name, repr(p.default), str(p.kind)) for p in inspect.signature(fn).parameters.values()]
+
+
+def state_dict_net(kind: str) -> O.Net:
+    cents = O.grid_centroids(2, 2) if kind == 'mega' else None
+    return O.make_net(kind, STATE_DICT_SPEC, seed=1, n_sub=4 if kind == 'mega' else 1, centroids=cents, cluster_2d=True)
+
+
+def case_cotangent(seed: int, rays, opts):
+    key = f'rgb_{"fine" if opts.fine_samples > 0 else "coarse"}'
+    return key, torch.randn(rays.shape[0], 3, generator=torch.Generator().manual_seed(seed))
 
 
 def random_case(seed: int):
@@ -62,69 +90,51 @@ def random_case(seed: int):
     return net, bg, rays, idx, opts, center, radius, rnd.random() < 0.5
 
 
-@pytest.mark.parametrize('seed', list(range(16)))
-def test_random_configuration_bit_exact(MG, seed):
+@pytest.mark.parametrize('seed', SEEDS)
+def test_random_configuration_bit_exact(live, seed):
     net, bg, rays, idx, opts, c, r, training = random_case(seed)
-    rn = MG.ref_net(net)
-    rb = MG.ref_net(bg) if bg is not None else None
-    for mod in (rn, rb):
-        if mod is not None:
-            mod.train(training)
-            for p in mod.parameters():
-                p.requires_grad_(True)
+    want = live['configurations'][seed]
     nt = dataclasses.replace(net, training=training)
     bt = dataclasses.replace(bg, training=training) if bg is not None else None
-    key = f'rgb_{"fine" if opts.fine_samples > 0 else "coarse"}'
-    cot = torch.randn(rays.shape[0], 3, generator=torch.Generator().manual_seed(seed))
-    torch.manual_seed(seed)
-    ref, rp = MG.R_render.render_rays(rn, rb, rays, idx, MG.hparams_of(opts), c, r, False, True, False)
-    (ref[key] * cot).sum().backward()
+    key, cot = case_cotangent(seed, rays, opts)
     torch.manual_seed(seed)
     got, gn, gb = O.render_grads(nt, bt, rays, idx, opts, c, r, {key: cot})
+    ref = want['results']
     assert set(got) == set(ref)
     for k in ref:
-        assert torch.equal(ref[k].detach(), got[k]), (seed, k, float((ref[k].detach() - got[k]).abs().max()))
-    sys.path.insert(0, os.path.join(C.ROOT, 'tests', 'golden'))
-    import make_golden_backward as MB
-    for mod, n_, g_ in ((rn, net, gn), (rb, bg, gb)):
-        if mod is None:
+        assert torch.equal(ref[k], got[k]), (seed, k, float((ref[k] - got[k]).abs().max()))
+    for tag, g_ in (('net', gn), ('bg', gb)):
+        if want['grads'][tag] is None:
+            assert g_ is None, (seed, tag)
             continue
-        for a, b in zip(MB.ref_grads(mod, n_), g_):
-            for k in a:
-                assert torch.equal(a[k], b[k]), (seed, k, float((a[k] - b[k]).abs().max()))
+        assert len(g_) == len(want['grads'][tag]), (seed, tag)
+        for a, b in zip(want['grads'][tag], g_):
+            assert set(a) == set(b), (seed, tag, set(a) ^ set(b))
+            for k, e in a.items():
+                flat = b[k].detach().reshape(-1)
+                assert tuple(b[k].shape) == e['shape'], (seed, tag, k)
+                sha = hashlib.sha256(b[k].detach().float().contiguous().numpy().tobytes()).hexdigest()
+                assert sha == e['sha256'], (seed, tag, k, float((flat[e['idx']] - torch.tensor(e['val'])).abs().max()))
 
 
-def test_call_surface_signatures_match_reference(MG):
+def test_call_surface_signatures_match_reference(live):
     """Drop-in boundary (SURVEY.md §8b): every replaced symbol takes the reference's parameters, in order, with the
     reference's defaults."""
-    import inspect
     import mega_nerf_b200 as M
-    from mega_nerf import ray_utils as R_rays, rendering as R_rendering
-    from mega_nerf.spherical_harmonics import eval_sh as R_eval_sh
-    from mega_nerf.models import nerf as R_nerf, mega_nerf as R_mega, cascade as R_cascade
-    pairs = [(M.render_rays, R_rendering.render_rays), (M.get_rays, R_rays.get_rays), (M.get_rays_batch, R_rays.get_rays_batch),
-             (M.get_ray_directions, R_rays.get_ray_directions), (M.eval_sh, R_eval_sh),
-             (M.NeRF.__init__, R_nerf.NeRF.__init__), (M.NeRF.forward, R_nerf.NeRF.forward),
-             (M.MegaNeRF.__init__, R_mega.MegaNeRF.__init__), (M.MegaNeRF.forward, R_mega.MegaNeRF.forward),
-             (M.Cascade.__init__, R_cascade.Cascade.__init__), (M.Cascade.forward, R_cascade.Cascade.forward),
-             (M.Embedding.__init__, R_nerf.Embedding.__init__), (M.ShiftedSoftplus.__init__, R_nerf.ShiftedSoftplus.__init__)]
-    for mine, ref in pairs:
-        a, b = inspect.signature(mine), inspect.signature(ref)
-        pa = [(p.name, p.default, p.kind) for p in a.parameters.values()]
-        pb = [(p.name, p.default, p.kind) for p in b.parameters.values()]
-        assert [x[0] for x in pa] == [x[0] for x in pb], (ref.__qualname__, pa, pb)
-        assert [x[1:] for x in pa] == [x[1:] for x in pb], (ref.__qualname__, pa, pb)
-    # model_utils needs configargparse-free import: compare by source inspection of the two factory signatures
-    import importlib
-    mu = importlib.import_module('mega_nerf.models.model_utils')
-    for name in ('get_nerf', 'get_bg_nerf'):
-        assert list(inspect.signature(getattr(M, name)).parameters) == list(inspect.signature(getattr(mu, name)).parameters)
+    surface = live['surface']
+    for mine_path, ref_path in SURFACE:
+        mine = M
+        for a in mine_path.split('.'):
+            mine = getattr(mine, a)
+        pa, pb = signature_of(mine), surface['signatures'][ref_path]
+        assert [x[0] for x in pa] == [x[0] for x in pb], (ref_path, pa, pb)
+        assert [x[1:] for x in pa] == [x[1:] for x in pb], (ref_path, pa, pb)
+    for name, params in surface['factories'].items():
+        assert list(inspect.signature(getattr(M, name)).parameters) == params, name
     # state-dict layout of every model family
-    spec = O.NerfSpec(layer_dim=32, appearance_count=5)
-    for kind in ('nerf', 'cascade', 'mega'):
-        cents = O.grid_centroids(2, 2) if kind == 'mega' else None
-        net = O.make_net(kind, spec, seed=1, n_sub=4 if kind == 'mega' else 1, centroids=cents, cluster_2d=True)
-        ref = MG.ref_net(net)
+    spec = STATE_DICT_SPEC
+    for kind in STATE_DICT_KINDS:
+        cents = state_dict_net(kind).centroids
         from test_host_factories import M as _M  # noqa: F401
         if kind == 'nerf':
             mine = M.NeRF(spec.pos_xyz_dim, spec.pos_dir_dim, spec.layers, list(spec.skip_layers), spec.layer_dim, spec.appearance_dim,
@@ -139,7 +149,8 @@ def test_call_surface_signatures_match_reference(MG):
                                 spec.appearance_dim, spec.affine_appearance, spec.appearance_count, spec.rgb_dim, spec.xyz_dim,
                                 M.ShiftedSoftplus())
             mine = M.MegaNeRF([mk() for _ in range(4)], cents, 1.15, False, True)
-        a, b = mine.state_dict(), ref.state_dict()
-        assert list(a) == list(b), (kind, set(a) ^ set(b))
-        assert all(a[k].shape == b[k].shape and a[k].dtype == b[k].dtype for k in b)
-        mine.load_state_dict(b)                      # reference checkpoints load
+        a, layout = mine.state_dict(), surface['state_dicts'][kind]
+        assert list(a) == [k for k, _, _ in layout], (kind, set(a) ^ {k for k, _, _ in layout})
+        assert all(tuple(a[k].shape) == s and str(a[k].dtype) == d for k, s, d in layout)
+        # reference checkpoints load: a state dict in the reference's layout
+        mine.load_state_dict({k: torch.zeros(s, dtype=getattr(torch, d.split('.')[-1])) for k, s, d in layout})
